@@ -23,6 +23,12 @@ merge (`qwgpu_response_to_partial` / `qwgpu_merge_partials`); times are the max 
 `--impl reference`: the reference's CPU algorithm (oracle/qw_oracle.c, a restatement — the real
 quickwit-search + tantivy cannot be built here, see DESIGN.md) on all host cores, one split per
 thread, on a bounded sample of the same workload.
+
+`--dump-outputs DIR`: what the last timed step of each region returned, as float64 DIR/<name>.npy (rank 0's
+view, at most 64 MB in all, a seeded sample of the rows beyond that): split_search_hits (query, split, doc id,
+score) and split_search_num_hits[query, split] from `value`; leaf_search_hits (query, split, doc id, sort value)
+and leaf_search_num_hits[query] from `e2e`. The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -67,7 +73,13 @@ def parse_args():
     ap.add_argument("--cpu-sample-splits", type=int, default=0, help="splits in the cpu_baseline sample (0 = auto)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-config block (C1 / C3 / C4)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
+    a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU arm (--impl qwgpu)")
+    return a
 
 
 MSG_VOCAB = 64  # vocabulary of the positions field "msg" (phrase queries of BASELINE config 5)
@@ -143,6 +155,49 @@ class RawSearch:
     def free(self):
         for i in range(self.n):
             self.L.qwgpu_split_result_free(C.byref(self.res[i]))
+
+
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much in all
+
+
+def sample_rows(a, max_bytes: int, seed: int = 0):
+    """`a` itself if it fits in max_bytes, else a fixed, seeded sample of its rows kept in their order."""
+    n = max_bytes // max(1, a[:1].nbytes)
+    if len(a) <= n:
+        return a
+    return a[np.sort(np.random.default_rng(seed).choice(len(a), n, replace=False))]
+
+
+def split_search_outputs(searches, split_gids):
+    """What qwgpu_split_search handed back in each search's latest run, before it is freed: hits rows
+    (query, split, doc id, BM25 score) in the order every split returned them, and num_hits[query, split]."""
+    rows, num_hits = [], np.zeros((len(searches), len(split_gids)))
+    for q, s in enumerate(searches):
+        for i in range(s.n):
+            r = s.res[i]
+            num_hits[q, i] = r.num_hits
+            if r.num_partial_hits:  # QwHit as eight u32: v1 (2), v2 (2), doc_id, flags, score (f32), reserved
+                h = np.ctypeslib.as_array(C.cast(r.hits, C.POINTER(C.c_uint32)), shape=(r.num_partial_hits, 8))
+                rows.append(np.stack([np.full(len(h), q), np.full(len(h), split_gids[i]), h[:, 4], h[:, 6].view(np.float32)], axis=1))
+    return (np.concatenate(rows) if rows else np.zeros((0, 4))), num_hits
+
+
+def leaf_search_outputs(resps, gid_of):
+    """The LeafSearchResponse of every query: partial-hit rows (query, split, doc id, sort value) and num_hits[query]."""
+    from quickwit_b200 import proto
+    rows, num_hits = [], np.zeros(len(resps))
+    for q, r in enumerate(resps):
+        d = proto.dec_leaf_search_response(r)
+        num_hits[q] = d["num_hits"]
+        rows += [(q, gid_of[h["split_id"]], h["doc_id"], h.get("sort_value", (None, np.nan))[1]) for h in d["partial_hits"]]
+    return np.array(rows, dtype=np.float64).reshape(-1, 4), num_hits
+
+
+def write_outputs(out_dir: str, arrays: dict):
+    os.makedirs(out_dir, exist_ok=True)
+    per_array = DUMP_BYTES // len(arrays) - 4096  # (room for the .npy header)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), sample_rows(a, per_array))
 
 
 class ClockSampler:
@@ -591,7 +646,7 @@ def main():
         gath_host = torch.zeros(world * Q_SETS * part_bytes, dtype=torch.uint8).pin_memory()
         by_query = torch.zeros(Q_SETS * world * part_bytes, dtype=torch.uint8)  # [query][rank][partial]
 
-    def step():
+    def step(keep: bool = False):
         acc = dict(gpu_us=0.0, main_us=0.0, launches=0, postings=0, alg_bytes=0, d2h=0, h2d=0, fallbacks=0)
         for s in searches:
             r = s.run()
@@ -600,7 +655,8 @@ def main():
             for k in ("launches", "postings", "alg_bytes", "d2h", "fallbacks"):
                 acc[k] += r[k]
             acc["h2d"] += s.plan_bytes
-            s.free()
+            if not keep:
+                s.free()
         return acc
 
     last = {}
@@ -681,9 +737,15 @@ def main():
         sampler.start()
     sync()
     t0 = time.perf_counter()
-    accs = [step() for _ in range(a.steps)]
+    # the last timed step's results are freed after the clock stops, so that --dump-outputs reads them
+    # without a copy inside the timed region
+    accs = [step(keep=i == a.steps - 1) for i in range(a.steps)]
     sync()
     wall_c = time.perf_counter() - t0
+    gids = [rank * a.splits + i for i in range(a.splits)]
+    split_out = split_search_outputs(searches, gids) if a.dump_outputs and rank == 0 else None
+    for s in searches:
+        s.free()
     for _ in range(max(a.warmup, 3)):
         step_e2e()
     sync()
@@ -711,6 +773,10 @@ def main():
         cold_ms = 1e3 * (time.perf_counter() - t)
     hits0 = proto.dec_leaf_search_response(last[0])
     assert len(hits0["partial_hits"]) == K and hits0["num_hits"] > 0
+    if split_out is not None:
+        leaf_out = leaf_search_outputs([last[q] for q in range(Q_SETS)], {f"bench-{g:04d}": g for g in range(world * a.splits)})
+        write_outputs(a.dump_outputs, {"split_search_hits": split_out[0], "split_search_num_hits": split_out[1],
+                                       "leaf_search_hits": leaf_out[0], "leaf_search_num_hits": leaf_out[1]})
 
     gpu_s = sum(x["gpu_us"] for x in accs) * 1e-6
     main_s = sum(x["main_us"] for x in accs) * 1e-6

@@ -27,7 +27,8 @@ def test_every_declared_symbol_is_exported():
 
 
 def test_no_cpu_fallback():
-    if os.path.exists("/dev/nvidia0"):
+    import torch
+    if torch.cuda.device_count() > 0:  # (asked of the CUDA runtime: a GPU's device node need not be /dev/nvidia0)
         pytest.skip("a GPU is present")
     with pytest.raises(ffi.QwGpuError) as e:
         service.SearcherContext(0)
@@ -395,6 +396,28 @@ def test_bench_reference_arm_prints_the_contract_line():
     assert d["value"] > 0 and d["steps"] == 2 and d["config"]["workload"] == "c2_bm25_or10_top1000"
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1 and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": "postings/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_refuses_arguments_it_cannot_honour():
+    """--steps below 1 would time nothing; --dump-outputs writes the outputs of the GPU arm only."""
+    import subprocess
+    import sys
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "unused"]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=120, cwd=ROOT)
+        assert out.returncode == 2 and "error:" in out.stderr, extra
+
+
+def test_bench_dump_sample_is_seeded_and_within_budget(tmp_path):
+    """Outputs larger than --dump-outputs' 64 MB are written as a fixed sample of their rows, in order."""
+    import bench
+    big = np.arange(12_000_000, dtype=np.float64).reshape(-1, 4)      # 96 MB
+    small = np.arange(8, dtype=np.float64)
+    bench.write_outputs(str(tmp_path / "a"), {"big": big, "small": small})
+    bench.write_outputs(str(tmp_path / "b"), {"big": big, "small": small})
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= bench.DUMP_BYTES
+    a, b = np.load(tmp_path / "a" / "big.npy"), np.load(tmp_path / "b" / "big.npy")
+    assert np.array_equal(a, b) and len(a) < len(big) and np.all(np.diff(a[:, 0]) > 0) and np.all(a[:, 0] % 4 == 0)
+    assert np.array_equal(np.load(tmp_path / "a" / "small.npy"), small)
 
 
 def test_wildcard_queries_expand_over_the_split_dictionary():
