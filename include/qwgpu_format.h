@@ -287,14 +287,24 @@ typedef struct QwHit {
 /* Dense aggregation result. Every QwAggNode owns `cells(node)` = Π num_buckets over its ancestor
  * chain (itself included; metric nodes count 1) cells, laid out row-major (outermost ancestor
  * slowest). Bucket nodes use only `count` (doc_count). Metric nodes (QW_AGG_STATS) use all four:
- * `sum_bits`: for integer-typed columns (u64, i64, datetime, bool) whose bit-packed raw width is at
- * most QW_SUM_EXACT_BITS, the exact integer sum of the RAW offsets (value = min_value + gcd * raw in
- * the mapped space) — the host rebuilds count * min + gcd * sum in 128-bit arithmetic, so e.g. an avg
- * over nanosecond timestamps cannot overflow; for f64 columns and wider raws, the bit pattern of an
- * f64 sum of the typed values (what tantivy accumulates). min/max are in the column's mapped-u64 space
- * (initialised to UINT64_MAX / 0). The host converts to f64 when it builds the intermediate
- * aggregation result. */
-#define QW_SUM_EXACT_BITS 40u /* 2^40 * 2^24 docs per split: the raw sum cannot wrap */
+ * `sum_bits`: for columns where qw_col_sum_exact() holds, the exact integer sum of the RAW offsets
+ * (value = min_value + gcd * raw in the mapped space) — the host rebuilds count * min + gcd * sum in
+ * 128-bit arithmetic, so e.g. an avg over nanosecond timestamps cannot overflow; for every other
+ * column, the bit pattern of an f64 sum of the typed values (what tantivy accumulates). min/max are
+ * in the column's mapped-u64 space (initialised to UINT64_MAX / 0). The host converts to f64 when it
+ * builds the intermediate aggregation result. */
+#define QW_SUM_EXACT_BITS 40u /* widest raw that may take the exact integer sum (see qw_col_sum_exact) */
+
+/* How a stats cell sums a column: 1 = exact uint64 sum of the raw offsets, 0 = f64 sum of the typed values.
+ * Exact only for integer-typed columns whose raws are at most QW_SUM_EXACT_BITS wide AND whose raws cannot
+ * wrap a uint64 when all of them are added: num_vals * (2^bits - 1) < 2^64. A cell sums a subset of the
+ * column's values, so the bound holds for every cell. The width alone is not enough: a multi-valued column
+ * holds more values than docs, and 2^24 values of 40 bits already reach 2^64. The oracle, the kernels (through
+ * DAgg::is_f64) and the host finalisation all decide with this one predicate. */
+static inline int qw_col_sum_exact(const QwImgColumn* c) {
+  if (c->type == QW_COL_F64 || c->bits > QW_SUM_EXACT_BITS) return 0;
+  return c->bits == 0 || c->num_vals <= UINT64_MAX / ((1ull << c->bits) - 1);
+}
 typedef struct QwAggCell {
   uint64_t count;
   uint64_t sum_bits;

@@ -564,7 +564,7 @@ static void agg_collect(Aggs* A, uint32_t ni, uint32_t doc, uint64_t parent_cell
     for (uint64_t i = a; i < b; i++) {
       uint64_t m = o_col_mapped(A->im, col, i);
       c->count++;
-      if (col->type == QW_COL_F64 || col->bits > QW_SUM_EXACT_BITS) {
+      if (!qw_col_sum_exact(col)) {
         /* tantivy: sum += value as f64, in doc order */
         double s; memcpy(&s, &c->sum_bits, 8); s += o_mapped_to_f64(col->type, m); memcpy(&c->sum_bits, &s, 8);
       } else {

@@ -447,7 +447,7 @@ static IAgg build_node(const BuildCtx& c, uint32_t ni, uint64_t parent_cell) {
     if (cell.count && b.column >= 0) {
       uint32_t t = b.col_type;
       const QwImgColumn& col = c.img.columns[b.column];
-      if (t == QW_COL_F64 || col.bits > QW_SUM_EXACT_BITS) memcpy(&a.m_sum, &cell.sum_bits, 8);
+      if (!qw_col_sum_exact(&col)) memcpy(&a.m_sum, &cell.sum_bits, 8);
       else {
         // exact: sum of the typed values = count * min + gcd * (sum of raw offsets); the mapped u64 of an
         // i64 / datetime is value + 2^63

@@ -70,7 +70,9 @@ struct DCol {  // 48 bytes
 struct DAgg {
   uint32_t kind, parent, first_child, num_children;
   uint32_t col, num_buckets, has_bounds, num_ranges;
-  uint32_t has_missing, cell_base, is_f64, pad;
+  uint32_t has_missing, cell_base;
+  uint32_t is_f64;  // STATS: 1 = the cell sums f64 values, 0 = exact u64 sum of raws (qw_col_sum_exact on the host)
+  uint32_t pad;
   double interval, offset, bound_min, bound_max;
   int64_t base_pos;
   // fast path (flat bucket aggregations over single-valued columns, see lower_plan): histogram

@@ -648,6 +648,7 @@ static void lower_plan(Lowered& L, const SplitDev& sp, const uint8_t* plan, size
     d.kind = a.kind; d.parent = a.parent; d.first_child = a.first_child; d.num_children = a.num_children;
     d.col = use_col(L, sp, a.column); d.num_buckets = a.num_buckets; d.has_bounds = a.has_bounds;
     d.num_ranges = a.num_ranges; d.has_missing = a.has_missing; d.cell_base = bases[i];
+    d.is_f64 = a.kind == QW_AGG_STATS && d.col != 0xFFFFFFFFu && !qw_col_sum_exact(&sp.view.columns[a.column]);
     d.interval = a.interval; d.offset = a.offset; d.bound_min = a.bound_min; d.bound_max = a.bound_max;
     d.base_pos = a.base_pos;
     memcpy(d.range_from, a.range_from, sizeof d.range_from);
@@ -678,8 +679,11 @@ static void lower_plan(Lowered& L, const SplitDev& sp, const uint8_t* plan, size
       d.stat_base = P.n_stat_cells;
       P.n_stat_cells += d.parent == 0xFFFFFFFFu ? 1u : L.aggs[d.parent].num_buckets;
     } else {
+      // a histogram's raw-space boundary table ends one past the largest raw; a column whose raws reach
+      // 2^64 - 1 has no such uint64 bound (its top value would fall outside the last bucket)
       if (d.parent != 0xFFFFFFFFu || (d.kind != QW_AGG_TERMS && d.kind != QW_AGG_HISTOGRAM) || !full_col ||
-          d.num_buckets > QW_SMEM_AGG_CELLS || d.num_buckets == 0)
+          d.num_buckets > QW_SMEM_AGG_CELLS || d.num_buckets == 0 ||
+          (d.kind == QW_AGG_HISTOGRAM && L.col_max_raw[d.col] == ~0ull))
         fast = false;
     }
   }
@@ -688,10 +692,9 @@ static void lower_plan(Lowered& L, const SplitDev& sp, const uint8_t* plan, size
     for (DAgg& d : L.aggs) {
       if (d.kind != QW_AGG_HISTOGRAM) continue;
       const DCol& c = L.cols[d.col];
-      // raws present in the column are <= max_raw; searching beyond would leave the value domain
+      // raws present in the column are < raw_end; searching beyond would leave the value domain
       // (f64 columns: bit patterns past the maximum are NaNs and break monotonicity)
-      const uint64_t max_raw = L.col_max_raw[d.col];
-      const uint64_t raw_end = max_raw == ~0ull ? max_raw : max_raw + 1;
+      const uint64_t raw_end = L.col_max_raw[d.col] + 1;  // < 2^64: checked above
       const uint32_t nb = d.num_buckets;
       // g(raw): bucket index clamped to [-1, nb]; monotone non-decreasing in raw
       auto g = [&](uint64_t raw) -> int64_t {
@@ -712,7 +715,6 @@ static void lower_plan(Lowered& L, const SplitDev& sp, const uint8_t* plan, size
       for (uint32_t k = 0; k <= nb; k++) {
         // smallest raw in [lo, raw_end] with g(raw) >= k (raw_end when there is none)
         uint64_t a = lo, b = raw_end;
-        if (max_raw == ~0ull && g(~0ull) < (int64_t)k) a = b = ~0ull;  // (2^64 is not representable: saturate)
         while (a < b) {
           const uint64_t mid = a + (b - a) / 2;
           if (g(mid) >= (int64_t)k) b = mid; else a = mid + 1;

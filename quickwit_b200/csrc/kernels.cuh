@@ -501,18 +501,16 @@ __device__ __forceinline__ uint64_t col_raw_doc(const uint8_t* base, const DCol&
   }
   return col_raw(base, c, doc);
 }
-// how a stats cell sums a column (also aggs.cpp build_node and the oracle)
-__device__ __forceinline__ bool stat_sum_f64(const DCol& c) { return c.type == QW_COL_F64 || c.bits > QW_SUM_EXACT_BITS; }
 // Privatised stats cell of the fast path: {sum (u64 wrapping, or f64 bits), max(~mapped) = min, max(mapped)}.
 // When the whole warp feeds one cell the three values are butterfly-reduced first.
-__device__ __forceinline__ void stat_update(unsigned long long* st, const DCol& c, const uint8_t* base, uint32_t cell, uint32_t doc, uint32_t num_docs, bool ok, uint32_t lane) {
+__device__ __forceinline__ void stat_update(unsigned long long* st, const DAgg& g, const DCol& c, const uint8_t* base, uint32_t cell, uint32_t doc, uint32_t num_docs, bool ok, uint32_t lane) {
   const uint32_t okmask = __ballot_sync(QW_FULL, ok);
   if (okmask == 0) return;
   const uint64_t raw = ok ? col_raw_doc(base, c, doc, num_docs) : 0ull;
   const uint64_t m = ok ? c.min_value + c.gcd * raw : 0ull;
   // sums: exact integer sum of the RAW offsets (the host rebuilds count * min + gcd * sum in 128 bits, so
-  // nanosecond timestamps cannot overflow); f64 columns and raws wider than QW_SUM_EXACT_BITS add doubles
-  const bool is_f64 = stat_sum_f64(c);
+  // nanosecond timestamps cannot overflow); other columns add doubles (qw_col_sum_exact, decided on the host)
+  const bool is_f64 = g.is_f64;
   unsigned long long isum = ok ? raw : 0ull;
   double dsum = (ok && is_f64) ? mapped_to_f64(c.type, m) : 0.0;
   unsigned long long nmin = ok ? ~m : 0ull, vmax = ok ? m : 0ull;
@@ -544,7 +542,7 @@ __device__ __forceinline__ void agg_collect_fast(const Sm& sm, const DSplitPlan&
     const DAgg& g = aggs[gi];
     if (g.parent != 0xFFFFFFFFu) continue;  // children are visited under their parent
     if (g.kind == QW_AGG_STATS) {
-      stat_update(st, cols[g.col], base, g.stat_base, doc, P.num_docs, on, lane);
+      stat_update(st, g, cols[g.col], base, g.stat_base, doc, P.num_docs, on, lane);
       continue;
     }
     const uint64_t raw = on ? col_raw_doc(base, cols[g.col], doc, P.num_docs) : 0ull;
@@ -569,7 +567,7 @@ __device__ __forceinline__ void agg_collect_fast(const Sm& sm, const DSplitPlan&
     else warp_count_few(ctr, g.cell_base + bk, ok, lane);
     for (uint32_t ci = 0; ci < g.num_children; ci++) {
       const DAgg& ch = aggs[g.first_child + ci];  // STATS over an always-present column
-      stat_update(st, cols[ch.col], base, ch.stat_base + bk, doc, P.num_docs, ok, lane);
+      stat_update(st, ch, cols[ch.col], base, ch.stat_base + bk, doc, P.num_docs, ok, lane);
     }
   }
 }
@@ -585,7 +583,7 @@ __device__ __forceinline__ void agg_stats(const DAgg& g, const DCol& c, const ui
   if (on) col_range(base, c, doc, a, b);
   const uint32_t nv = (uint32_t)(b - a);
   const uint32_t maxv = __reduce_max_sync(QW_FULL, nv);
-  const bool is_f64 = stat_sum_f64(c);
+  const bool is_f64 = g.is_f64;
   for (uint32_t k = 0; k < maxv; k++) {
     const bool ok = k < nv;
     const uint32_t okmask = __ballot_sync(QW_FULL, ok);
@@ -1443,7 +1441,7 @@ __global__ void __launch_bounds__(QW_THREADS, QW_MIN_BLOCKS_PER_SM) k_window(con
           if (g.kind != QW_AGG_STATS) continue;
           const bool top = g.parent == 0xFFFFFFFFu;
           const uint32_t nc = top ? 1u : s_aggs[g.parent].num_buckets;
-          const bool is_f64 = stat_sum_f64(s_cols[g.col]);
+          const bool is_f64 = g.is_f64;
           for (uint32_t c = tid; c < nc; c += QW_THREADS) {
             const uint32_t cnt = top ? s_misc[2] : s_hist[s_aggs[g.parent].cell_base + c];
             if (!cnt) continue;
